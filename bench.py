@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — image-pairs/sec of the MicKey inference hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Default workload (config.workload): BASELINE configs[2], the largest single-GPU configuration — a batch of 32
@@ -27,6 +27,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -253,10 +254,9 @@ def run_reference_arm(args, wl):
     if rank != 0:
         return
     threads = cpu_threads()
-    # a "step" is one pair of the workload's configuration through the CPU path; the run is bounded
-    steps, warm = max(1, min(args.steps, 6)), max(0, min(args.warmup, 1))
-    durs = cpu_reference_run(wl, steps, warm, threads, budget_s=150.0)
-    steps = len(durs)
+    # a "step" is one pair of the workload's configuration through the CPU path
+    steps, warm = args.steps, max(0, min(args.warmup, 1))
+    durs = cpu_reference_run(wl, steps, warm, threads, budget_s=float("inf"))
     val = len(durs) / sum(durs)
     line = {"impl": "reference", "metric": "image-pairs/sec @720x540", "value": val, "unit": "pairs/s", "n_gpus": args.gpus,
             "steps": steps, "warmup": warm, "ms_per_step": 1e3 * sum(durs) / len(durs), "higher_is_better": True,
@@ -264,7 +264,7 @@ def run_reference_arm(args, wl):
             "config": {"workload": wl[4], "note": "reference CPU path (oracle port of the PyTorch reference), rank 0 only; "
                                                   "each step = ONE pair of the workload's model / hypothesis configuration"},
             "cpu_baseline": {"value": val, "unit": "pairs/s", "cores": threads, "kind": "port",
-                             "sample": f"{steps} pair(s) of the workload's configuration (steps clamped to 6 / 150 s, {warm} warm-up), "
+                             "sample": f"{steps} pair(s) of the workload's configuration ({warm} warm-up), "
                                        f"torch threads = {threads} of {usable_cpus()} usable"},
             "e2e": {"value": val, "unit": "pairs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line), flush=True)
@@ -293,7 +293,9 @@ class Runner:
         data = dict(self.dev_data)
         R, t = self.model(data)
         packed = torch.cat([R.reshape(B, 9), t.reshape(B, 3), data["inliers"].reshape(B, 1)], dim=1)
-        return self.mkdist.gather_poses(packed)
+        poses = self.mkdist.gather_poses(packed)
+        self.last = (data, poses)
+        return poses
 
     def step_e2e(self):
         # pinned HOST images go straight into model(): the engine's H2D copies land in its static input buffer
@@ -347,6 +349,25 @@ class Runner:
         return {"median_ms": mx[len(mx) // 2], "min_ms": mx[0], "max_ms": mx[-1], "own_median_ms": own[len(own) // 2], "n": n_blocks}
 
 
+def snapshot_outputs(data, poses, n_cols=256, n_cells=1 << 18):
+    """What the caller of a step receives, as float32 host arrays: the gathered [B,13] poses, R, t, inliers and the
+    per-keypoint outputs in full; the descriptors and the three N x N score tensors (480 MB each at B = 32) as a fixed
+    seeded sample of keypoint columns / cells, the same for every run of a workload."""
+    dev = data["dsc0"].device
+    B, _, N = data["dsc0"].shape
+    g = torch.Generator().manual_seed(0)
+    cols = torch.randperm(N, generator=g)[:n_cols].sort().values.to(dev)
+    b, i, j = (torch.randint(n, (n_cells,), generator=g).to(dev) for n in (B, N, N))
+    out = {"poses": poses}
+    for k in ("R", "t", "inliers", "kps0", "kps1", "depth_kp0", "depth_kp1", "scr0", "scr1"):
+        out[k] = data[k]
+    for k in ("dsc0", "dsc1"):
+        out[k + "_sample"] = data[k][:, :, cols]
+    for k in ("scores", "kp_scores", "final_scores"):
+        out[k + "_sample"] = data[k][b, i, j]
+    return {k: v.float().cpu().numpy() for k, v in out.items()}
+
+
 def stats(blk, steps, pairs_per_step_all_ranks):
     return {"value": pairs_per_step_all_ranks * steps / (blk["median_ms"] / 1e3), "ms_per_step": blk["median_ms"] / steps,
             "ms_per_step_min": blk["min_ms"] / steps, "ms_per_step_max": blk["max_ms"] / steps, "blocks": blk["n"]}
@@ -355,7 +376,7 @@ def stats(blk, steps, pairs_per_step_all_ranks):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="steps in each timed block")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS),
@@ -366,7 +387,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--no-c2", action="store_true", help="skip the latency_c2 object of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, float32, ~14 MB for c3; "
+                         "the inputs are seeded, so two builds run with the same arguments can be compared file by file")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference_arm(args, wl)
@@ -383,10 +411,10 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     torch.manual_seed(1234 + rank)
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)     # > 126 MB L2
-    lat_steps = max(1, min(args.steps, 10))
 
-    def measure(wl_, depth, n_blocks, with_profile=True):
-        """Full measurement of one workload: single-step latency, pipelined throughput, e2e, per-kernel profile."""
+    def measure(wl_, depth, n_blocks, with_profile=True, dump=False):
+        """Full measurement of one workload: single-step latency, pipelined throughput, e2e, per-kernel profile.
+        dump: also return the outputs of the last timed throughput step (snapshot_outputs)."""
         r = Runner(wl_, dev, rank, world)
         model, B = r.model, r.B
         # (1) latency: one step at a time (pipeline depth 1), L2 flushed between steps
@@ -397,7 +425,7 @@ def main():
         if ncu_range:
             torch.cuda.synchronize()
             torch.cuda.profiler.start()
-        lat = r.blocks(r.step_device, lat_steps, 3, flush)
+        lat = r.blocks(r.step_device, args.steps, 3, flush)
         if ncu_range:
             torch.cuda.synchronize()
             torch.cuda.profiler.stop()
@@ -415,6 +443,7 @@ def main():
         dev_blk = r.blocks(r.step_device, args.steps, n_blocks)
         launches = (sum(e.total_kernel_launches for e in engines) - l0) // n_blocks
         clock_info = clocks.finish() if rank == 0 else None
+        outputs = snapshot_outputs(*r.last) if dump else None      # before the e2e steps overwrite the static outputs
         ws_bytes = sum(int(e.ws.numel()) for e in engines)
         for _ in range(4 * max(1, depth)):
             r.step_e2e()
@@ -443,16 +472,18 @@ def main():
             eng.profile(False)
             prof = {k: {"scopes_per_step": v[0] / n_prof, "ms_per_step": v[1] / n_prof} for k, v in raw.items()}
         out = dict(B=B, lat=lat, dev=dev_blk, e2e=e2e_blk, launches=int(launches), clocks=clock_info, ws_bytes=ws_bytes,
-                   prof=prof, spread=spread, depth=max(1, depth))
+                   prof=prof, spread=spread, depth=max(1, depth), outputs=outputs)
         del r, model, eng, engines
         torch.cuda.empty_cache()
         return out
 
     depth = args.depth or (1 if args.workload == "c3" else 3)
     n_blocks = args.blocks or (5 if args.workload == "c3" else 9)
-    if args.workload == "c1":
-        args.steps = min(args.steps, 20)
-    m = measure(wl, depth, n_blocks)
+    m = measure(wl, depth, n_blocks, dump=bool(args.dump_outputs) and rank == 0)
+    if m["outputs"] is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in m["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
     c2 = None
     if args.workload == "c3" and world == 1 and not args.no_c2:
         c2 = measure(WORKLOADS["c2"], 3, 9, with_profile=True)
@@ -535,7 +566,7 @@ def main():
         "metric": "image-pairs/sec @720x540", "value": dev_s["value"], "unit": "pairs/s", "n_gpus": world, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": dev_s["ms_per_step"], "ms_per_step_min": dev_s["ms_per_step_min"],
         "ms_per_step_max": dev_s["ms_per_step_max"], "blocks": dev_s["blocks"],
-        "latency_ms_single_step": m["lat"]["median_ms"] / lat_steps,
+        "latency_ms_single_step": m["lat"]["median_ms"] / args.steps,
         "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f16 operands / f32 accumulate (tensor core), f32 matcher+solver", "data": "synthetic",
         "config": {"workload": wl[4] + (f"; {world} GPUs = BASELINE configs[3] (B={world * B} sharded {B} pairs per GPU, NCCL gather of poses)"
@@ -573,7 +604,7 @@ def main():
         d2, e2 = stats(c2["dev"], args.steps, c2["B"]), stats(c2["e2e"], args.steps, c2["B"])
         line["latency_c2"] = {"workload": WORKLOADS["c2"][4], "value": d2["value"], "unit": "pairs/s", "ms_per_step": d2["ms_per_step"],
                               "ms_per_step_min": d2["ms_per_step_min"], "ms_per_step_max": d2["ms_per_step_max"], "blocks": d2["blocks"],
-                              "latency_ms_single_step": c2["lat"]["median_ms"] / lat_steps, "steps_in_flight": c2["depth"],
+                              "latency_ms_single_step": c2["lat"]["median_ms"] / args.steps, "steps_in_flight": c2["depth"],
                               "e2e": {"value": e2["value"], "ms_per_step": e2["ms_per_step"], "h2d_bytes_per_step": int(2 * 3 * H_IMG * W_IMG * 4),
                                       "d2h_bytes_per_step": 52}, "gpu_launches": c2["launches"],
                               "stage_ms": {k: round(v["ms_per_step"], 4) for k, v in sorted(c2["prof"].items(), key=lambda kv: -kv[1]["ms_per_step"])}}

@@ -1,6 +1,7 @@
 """CPU tests of the Map-free loader side (SURVEY.md §8 f3): scene parsing, pair enumeration, rank sharding, the uint8
-batch variant, and — when the reference tree is present — item-by-item equality with the reference's own dataset on a
-generated tree."""
+batch variant, and item-by-item equality with the reference's own dataset on a generated tree."""
+import hashlib
+import json
 import os
 import sys
 
@@ -19,8 +20,6 @@ from lib.datasets.sampler import ShardedSequentialSampler            # noqa: E40
 from lib.datasets.utils import correct_intrinsic_scale               # noqa: E402
 from mickey_b200.io import to_float_chw, from_float_chw              # noqa: E402
 from tools.make_synthetic_mapfree import make_tree                   # noqa: E402
-
-REF = "/root/reference"
 
 
 @pytest.fixture(scope="module")
@@ -75,36 +74,35 @@ def test_rank_sharding_covers_every_pair_once(tree):
         DataModule(cfg).train_dataloader()
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "lib", "datasets", "mapfree.py")), reason="reference tree not present")
 def test_items_equal_the_reference_dataset(tree):
-    cfg = _cfg_for(tree)
-    ours = MapFreeDataset(cfg, "val")
-    saved = {k: v for k, v in sys.modules.items() if k == "lib" or k.startswith("lib.")}
-    for k in saved:
-        del sys.modules[k]
-    sys.path.insert(0, REF)
-    try:
-        import lib.datasets.mapfree as ref_mapfree
-        assert ref_mapfree.__file__.startswith(REF)
-        theirs = ref_mapfree.MapFreeDataset(cfg, "val")
-        assert len(theirs) == len(ours)
-        # the reference lists the scenes in directory order (mapfree.py:178), ours are sorted (every rank must build
-        # the same pair list): match the items by (scene, pair)
-        ref_items = {(b["scene_id"], b["pair_id"]): b for b in (theirs[i] for i in range(len(theirs)))}
-        for i in range(len(ours)):
-            a = ours[i]
-            b = ref_items[(a["scene_id"], a["pair_id"])]
-            assert set(a) == set(b)
-            for k in a:
+    """Item-by-item equality with the reference's own dataset (lib/datasets/mapfree.py) on the same generated tree, as
+    recorded by tests/golden/make_reference_fixtures.py: images by the SHA-256 of their float32 bytes (and a fixed
+    sample of values), every other field in full."""
+    with open(os.path.join(ROOT, "tests", "golden", "reference_mapfree_items.json")) as f:
+        theirs = json.load(f)
+    ours = MapFreeDataset(_cfg_for(tree), "val")
+    assert len(theirs) == len(ours)
+    # the reference lists the scenes in directory order (mapfree.py:178), ours are sorted (every rank must build
+    # the same pair list): match the items by (scene, pair)
+    ref_items = {(b["scene_id"]["value"], b["pair_id"]["value"]): b for b in theirs}
+    for i in range(len(ours)):
+        a = ours[i]
+        b = ref_items[(a["scene_id"], a["pair_id"])]
+        assert set(a) == set(b)
+        for k in a:
+            if "image" in b[k]:
+                img, rec = a[k].numpy(), b[k]["image"]
+                assert list(img.shape) == rec["shape"] and img.dtype == np.float32, k
+                assert img.reshape(-1)[rec["sample_idx"]].tolist() == rec["sample"], k
+                assert hashlib.sha256(np.ascontiguousarray(img).tobytes()).hexdigest() == rec["sha256"], k
+            elif "array" in b[k]:
+                ref = np.array(b[k]["array"], dtype=b[k]["dtype"])
                 if torch.is_tensor(a[k]):
-                    assert torch.equal(a[k], torch.as_tensor(b[k])), k
-                elif isinstance(a[k], np.ndarray):
-                    assert np.array_equal(a[k], np.asarray(b[k])), k
+                    assert torch.equal(a[k], torch.as_tensor(ref)), k
                 else:
-                    assert a[k] == b[k], k
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k == "lib" or k.startswith("lib.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
+                    assert isinstance(a[k], np.ndarray) and np.array_equal(a[k], ref), k
+            elif "relpath" in b[k]:
+                assert os.path.relpath(a[k], tree) == b[k]["relpath"], k
+            else:
+                ref = tuple(b[k]["value"]) if b[k]["tuple"] else b[k]["value"]
+                assert a[k] == ref, k

@@ -1,10 +1,12 @@
 """CPU tests of the host-side logic: config tree, state-dict naming, weight packing, C-ABI exports."""
 import ctypes
+import json
 import os
 import re
 
 import pytest
 import torch
+import yaml
 
 from mickey_b200 import _lib
 from mickey_b200.config import default_cfg, mickey_cfg, backbone_variant, CfgNode
@@ -26,11 +28,15 @@ def test_cfg_tree_access_and_merge(tmp_path):
     assert isinstance(cfg.clone(), CfgNode)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/config"), reason="reference tree not present")
-def test_reference_yaml_merges():
-    for f in ("curriculum_learning.yaml", "overlap_score.yaml"):
+def test_reference_yaml_merges(tmp_path):
+    """The reference's released configs (config/MicKey/*.yaml, stored as parsed in tests/golden) merge into ours."""
+    with open(os.path.join(ROOT, "tests", "golden", "reference_configs.json")) as fh:
+        configs = json.load(fh)
+    assert sorted(configs) == ["curriculum_learning.yaml", "overlap_score.yaml"]
+    for f, content in configs.items():
+        (tmp_path / f).write_text(yaml.safe_dump(content))
         cfg = default_cfg()
-        cfg.merge_from_file(f"/root/reference/config/MicKey/{f}")
+        cfg.merge_from_file(str(tmp_path / f))
         assert cfg.PROCRUSTES.NUM_SAMPLED_MATCHES == 2048
         assert backbone_variant(cfg) == "vitl"
         make_mk_config(cfg)

@@ -1,17 +1,29 @@
 """Pins the CPU oracle (oracle/mickey_oracle.py) to outputs of the unmodified reference.
 
-The committed fixtures were produced by tests/golden/make_golden.py from /root/reference; these
-tests re-create the seeded inputs/weights, run the oracle and compare.  When the reference tree is
-present (build container) one extra test runs the reference live next to the oracle.
+The committed fixtures were produced by tests/golden/make_golden.py and make_reference_fixtures.py from the
+reference; these tests re-create the seeded inputs/weights, run the oracle and compare.
 """
+import contextlib
+
 import pytest
 import torch
 
 from mickey_b200.config import mickey_cfg
 from mickey_b200.weights import synthetic_state_dict
 from oracle import mickey_oracle as mo
-from oracle import ref_harness
 from tests.common import GOLDEN_CASES, load_golden, synthetic_pair, rel_err, rotation_angle_deg
+
+
+@contextlib.contextmanager
+def _threads(n):
+    """Run torch CPU ops on n threads: how many threads split a reduction moves fp32 results by a few 1e-6, and with
+    them the draws of torch.multinomial."""
+    old = torch.get_num_threads()
+    torch.set_num_threads(n)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(old)
 
 
 def _run_oracle(name, inject=True):
@@ -58,22 +70,20 @@ def test_oracle_same_rng_stream_as_reference():
     data = synthetic_pair(spec["batch"], spec["height"], spec["width"], seed=spec["data_seed"])
     trace = {}
     torch.manual_seed(spec["rng_seed"])
-    with torch.no_grad():
+    # the recorded draws are reproduced with 2 to 8 threads; 1 or 16 threads move a few of the 16384 outer draws
+    with torch.no_grad(), _threads(8):
         mo.model_forward(sd, data, cfg, trace=trace)
     assert torch.equal(trace["outer_idx"].int(), gold["outer_idx"])
     assert torch.equal(trace["inner_idx"].to(torch.int16), gold["inner_idx"])
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not ref_harness.available(), reason="reference tree not present")
 def test_oracle_matches_live_reference_stagewise():
+    """compute_matches() of the reference, recorded by tests/golden/make_reference_fixtures.py, next to the oracle."""
     cfg = mickey_cfg("vits", 2, 8, float16=False)
     sd = synthetic_state_dict(cfg, seed=2)
-    model = ref_harness.build_reference_model(cfg, sd, variant="vits")
     data = synthetic_pair(1, 154, 140, seed=9)
-    ref = dict(data)
-    with torch.no_grad():
-        model.compute_matches(ref)
+    ref = load_golden("reference_stagewise_vits")
+    with torch.no_grad(), _threads(1):           # recorded on one thread
         ours = mo.compute_correspondences(sd, data, cfg)
     for k in ("kps0", "depth_kp0", "scr0", "dsc0", "scores", "kp_scores"):
         assert rel_err(ours[k], ref[k]) < 1e-6, k
